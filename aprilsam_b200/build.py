@@ -91,16 +91,8 @@ def build(force: bool = False, verbose: bool = False) -> str:
         _run([CC, "-std=gnu99", "-O2", "-g", "-I" + os.path.join(ROOT, "include", "aprilsam"), "-o", REPLAY_CLI, csrc,
               "-L" + LIB_DIR, "-laprilsam_b200", "-Wl,-rpath," + LIB_DIR, "-Wl,-rpath,$ORIGIN/../../aprilsam_b200/lib",
               "-lm"], log)
-    # the reference's own example programs, UNCHANGED, linked against this library (drop-in proof, run by
-    # the GPU tests); only where the reference sources exist -- binaries only, git-ignored like oracle/_ref
-    ref_ex = "/root/reference/examples"
-    if os.path.isdir(ref_ex):
-        for name in ("aprilsam_tutorial", "aprilsam_demo", "aprilsam_graph_save_simple", "aprilsam_graph_save_with_attributes"):
-            src, out = os.path.join(ref_ex, name + ".c"), os.path.join(os.path.dirname(REPLAY_CLI), "ref_" + name)
-            if os.path.exists(src) and (force or _stale(out, [src, LIB] + hdrs)):
-                _run([CC, "-std=gnu99", "-O2", "-w", "-I" + os.path.join(ROOT, "include"), "-o", out, src, "-L" + LIB_DIR,
-                      "-laprilsam_b200", "-Wl,-rpath," + LIB_DIR, "-Wl,-rpath,$ORIGIN/../../aprilsam_b200/lib", "-lm"], log)
-    # the oracle: C restatement always; the real reference only where its sources exist
+    # the oracle: C restatement always; the real reference and its example programs (linked against this
+    # library) only where the reference sources exist
     _run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "all"], log)
     with open(os.path.join(LIB_DIR, "build.log"), "w") as f:
         f.write("\n".join(log))

@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--workload all|manhattan_batch|m3500_batch|m3500_replay|manhattan_replay]
-                    [--poses P] [--replay-from S] [--shard auto|on|off]
+                    [--poses P] [--replay-from S] [--shard auto|on|off] [--dump-outputs DIR]
 
 One "step" is one pass of the hot path over one batch of synthetic/fixture input:
   *_batch   one april_graph_cholesky() call on the full graph (relinearise -> assemble ->
@@ -37,6 +37,14 @@ segments, the top of the tree replicated -- DESIGN.md section 6): every rank cal
 on its copy of the graph, value = solves / max rank time, scaling "strong", and the line carries
 `parity.sharded_vs_single_gpu_max_rel`.  M3500 and every incremental workload do not shard (SURVEY.md
 section 8e "replicas only"): each rank runs its own replica, value = total solves / max rank time.
+
+--dump-outputs DIR (rank 0) writes, after the timed steps, what the last timed step of every workload
+handed its caller, as float64 DIR/<workload>_<array>.npy:
+  *_batch   states   node states after the last timed april_graph_cholesky call (N x 3, node order)
+            step     Gauss-Newton step of the last device-resident pipeline step (N x 3, elimination order)
+  *_replay  states   node states after the last timed april_graph_cholesky_inc call
+The inputs are seeded, so two builds run with the same arguments can be compared array for array.  Above
+64 MiB in all, every array keeps the same fixed, seeded fraction of its rows.
 """
 from __future__ import annotations
 
@@ -59,6 +67,7 @@ from aprilsam_b200 import harness as H  # noqa: E402
 METRIC = "Gauss-Newton solves/sec (batch + incremental) on M3500 & 100k-pose graph"
 ALL = ["manhattan_batch", "m3500_batch", "m3500_replay", "manhattan_replay"]
 MIN_TIMED_S = 1.0  # sub-workloads: timed region at least this long
+DUMP_MAX_BYTES = 64 << 20
 
 
 def load_workload(name: str, poses: int):
@@ -401,6 +410,7 @@ def bench_batch(ctx: Ctx, name: str, d, label: str, K: int, W: int, sharded: boo
     launches1, h2d1, d2h1 = capi.counters(dev)
     e2e_val = aggregate_rate(dist, local, jobs, len(e2e_ms), float(np.sum(e2e_ms)) / 1e3)
     kern = np.array(kern)
+    e2e_states = h.states()
 
     # ---- e2e with the plan rebuilt on every call (ordering + symbolic, like the reference) ---------
     n_unc = max(3, min(K, int(1.0 / max(cold_ms * 1e-3, 1e-3)) + 3)) if not sharded else 3
@@ -444,6 +454,8 @@ def bench_batch(ctx: Ctx, name: str, d, label: str, K: int, W: int, sharded: boo
     L.asam_factor_status(dev, C.byref(st))
     if st.value != 0:
         raise SystemExit(f"bench.py: factorisation status {st.value}")
+    step = np.empty((N, 3), dtype=np.float64)
+    capi.check(L.asam_download_x(dev, 0, N, step.ctypes.data_as(C.POINTER(C.c_double))), "asam_download_x")
     value = aggregate_rate(dist, local, jobs, len(dev_ms), float(np.sum(dev_ms)) / 1e3)
     h.close()
 
@@ -474,6 +486,7 @@ def bench_batch(ctx: Ctx, name: str, d, label: str, K: int, W: int, sharded: boo
         rec["parity"] = {"vs_reference_first_iteration_max_rel": float(np.abs(first_states - ref_first).max() / scale),
                          "tolerance": 1e-6}
     rec["_first_states"] = first_states
+    rec["_outputs"] = {"states": e2e_states, "step": step}
     return rec
 
 
@@ -533,7 +546,21 @@ def bench_replay(ctx: Ctx, name: str, d, label: str, K: int, W: int, with_cpu: b
                                                        "aprilsam.c:556-559 active; non-deterministic, speed reference only)"}
     rec["_chi2_end"] = chi2_end
     rec["_end_states"] = end_states
+    rec["_outputs"] = {"states": end_states}
     return rec
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """DIR/<name>.npy in float64; above DUMP_MAX_BYTES in all, the same seeded fraction of every array's rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.size * 8 for a in arrays.values())
+    frac = min(1.0, DUMP_MAX_BYTES / max(total, 1))
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if frac < 1.0:
+            keep = np.sort(np.random.default_rng(0).choice(len(a), size=int(len(a) * frac), replace=False))
+            a = a[keep]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_b200(args, names, world, rank, local, dist):
@@ -582,6 +609,8 @@ def run_b200(args, names, world, rank, local, dist):
     clocks = sampler.stop() if rank == 0 else {}
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {f"{n}_{k}": v for n, r in recs.items() for k, v in r["_outputs"].items()})
     for r in recs.values():
         for k in [k for k in r if k.startswith("_")]:
             del r[k]
@@ -621,6 +650,8 @@ def main():
     ap.add_argument("--poses", type=int, default=100000)
     ap.add_argument("--replay-from", type=int, default=50000, help="manhattan_replay: first timed step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the arrays the last timed step of every workload computed as DIR/<workload>_<array>.npy")
     ap.add_argument("--shard", choices=["auto", "on", "off"], default="auto",
                     help="--gpus N > 1: shard the elimination tree of ONE solve over the GPUs (NCCL) instead of "
                          "running N replicas; auto = on for manhattan_batch (SURVEY.md section 8e)")
